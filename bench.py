@@ -22,8 +22,9 @@ reconstruction (stage 2).
          to the CPUs of its GPU's NUMA node first (pinned rings are then node-local).
   verified  after the timed region the LAST picture of every stream of the rank (60 pictures deep into
          the P chains) is read back and its FNV-1a hash compared with the unmodified reference C
-         (oracle/_ref) decoding the same stream on the host; the run FAILS (exit 1) on any difference
-         or if any picture fell back from the lane-parallel walk.
+         (oracle/_ref; where that was not built, the oracle, pinned to it by the tests) decoding the same
+         stream on the host; the run FAILS (exit 1) on any difference or if any picture fell back from the
+         lane-parallel walk.
   roofline  stage-2 kernel: algorithmic bytes (DESIGN.md) / CUDA-event time of its launches on the
          stream they run on; in the value leg nothing else runs beside them.
   cpu_baseline  oracle/_ref (the unmodified reference C, compiled in place) on the host cores this
@@ -52,6 +53,8 @@ import subprocess
 import sys
 import threading
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "tools")):
@@ -269,15 +272,38 @@ def run_reference_cpu(clips, threads, loops):
     return sum(counts), max(spent), "port"
 
 
+def oracle_last_hash(lib, es):
+    """(pictures, hash of the LAST picture) of one clip decoded by the oracle through the 15-function ABI."""
+    d = lib.mpeg1_decoder_create(len(es) + 16, 2)
+    ctypes.memmove(lib.mpeg1_decoder_get_write_ptr(d, len(es)), es, len(es))
+    lib.mpeg1_decoder_did_write(d, len(es))
+    n = 0
+    while lib.mpeg1_decoder_decode(d):
+        n += 1
+    ysz = lib.mpeg1_decoder_get_coded_size(d)
+    h = 1469598103934665603
+    for ptr, size in ((lib.mpeg1_decoder_get_y_ptr(d), ysz), (lib.mpeg1_decoder_get_cr_ptr(d), ysz >> 2),
+                      (lib.mpeg1_decoder_get_cb_ptr(d), ysz >> 2)):
+        h = lib.oracle_hash_bytes(h, ptr, size)
+    lib.mpeg1_decoder_destroy(d)
+    return n, int(h) if n > 0 else None
+
+
 def reference_last_hashes(clips, workers):
-    """hash of the LAST picture of each clip, decoded by the reference on `workers` host threads."""
+    """(pictures, hash of the LAST picture) of each clip, decoded on `workers` host threads by the reference
+    (oracle/_ref) or, where that was not built, by the oracle, which the test suite pins to the reference."""
     lib = ref_library()
+    olib = None
     if lib is None:
-        return None
+        olib = oracle_library()
+        olib.mpeg1_decoder_destroy(olib.mpeg1_decoder_create(16, 2))  # its VLC tables are built once, here
     out = [None] * len(clips)
 
     def work(k):
         for c in range(k, len(clips), workers):
+            if olib is not None:
+                out[c] = oracle_last_hash(olib, clips[c])
+                continue
             buf = (ctypes.c_uint64 * (PICTURES + 4))()
             n = lib.ref_picture_hashes(clips[c], len(clips[c]), buf, PICTURES + 4)
             out[c] = (int(n), int(buf[min(n, PICTURES + 4) - 1]) if n > 0 else None)
@@ -290,13 +316,29 @@ def reference_last_hashes(clips, workers):
     return out
 
 
+_oracle = None
+
+
+def oracle_library():
+    """oracle/liboracle.so: our CPU restatement of the reference (built by build()); here for its FNV-1a 64."""
+    global _oracle
+    if _oracle is None:
+        from jsmpeg_b200 import capi
+        lib = capi.load_library(os.path.join(ROOT, "oracle", "liboracle.so"))
+        lib.oracle_hash_bytes.restype = ctypes.c_uint64
+        lib.oracle_hash_bytes.argtypes = [ctypes.c_uint64, ctypes.c_void_p, ctypes.c_size_t]
+        _oracle = lib
+    return _oracle
+
+
 def fnv1a64_planes(y, cr, cb):
-    """FNV-1a 64 of Y | Cr | Cb exactly as oracle/ref_bench.c computes it (the hash is inherently serial;
-    Python ints would take seconds per picture, so the byte loop runs in the same C: ref_hash_bytes)."""
-    lib = ref_library()
+    """FNV-1a 64 of Y | Cr | Cb, the hash oracle/ref_bench.c gives the reference's pictures (the hash is inherently
+    serial; Python ints would take seconds per picture, so the byte loop runs in C: oracle_hash_bytes)."""
+    lib = oracle_library()
     h = 1469598103934665603
     for a in (y, cr, cb):
-        h = lib.ref_hash_bytes(h, a.ctypes.data, a.size)
+        a = np.ascontiguousarray(a)
+        h = lib.oracle_hash_bytes(h, a.ctypes.data, a.size)
     return int(h)
 
 
@@ -425,8 +467,6 @@ class Legs:
     def verify(self, seeds, workers):
         """The last picture of every stream, as the value leg left it in HBM, against the reference's
         decode of the same stream (FNV-1a 64 over Y | Cr | Cb).  Returns a dict for the JSON line."""
-        if ref_library() is None:
-            return {"verified": None, "why": "oracle/_ref not built on this box"}
         # distinct clips only once on the host
         uniq = {}
         for i, s in enumerate(seeds):
@@ -443,7 +483,30 @@ class Legs:
                 if n_ref != PICTURES or fnv1a64_planes(y, cr, cb) != h_ref:
                     bad.append(i)
         return {"verified": not bad, "streams_checked": checked, "pictures_deep": PICTURES, "mismatching_streams": bad[:16],
-                "checker": "oracle/_ref (unmodified reference C) on the host, FNV-1a 64 of Y|Cr|Cb of each stream's last picture"}
+                "checker": ("oracle/_ref (unmodified reference C)" if ref_library() is not None else "oracle (C restatement of the reference)")
+                           + " on the host, FNV-1a 64 of Y|Cr|Cb of each stream's last picture"}
+
+
+DUMP_BYTES = 56 << 20  # the sampled planes; with their positions < 64 MB in all
+
+
+def dump_outputs(directory, legs, prefix=""):
+    """What the value leg's last step left for its caller: per stream the Y / Cr / Cb planes of its last picture
+    (jsmpeg_b200_batch_read_planes).  All of them would be ~200 MB at 64 x 1080p, so every stream's planes are
+    sampled at the same fixed, seeded positions: <name>.npy is float32 [streams, samples], <name>_positions.npy the
+    sample positions in the plane (float64)."""
+    os.makedirs(directory, exist_ok=True)
+    planes = [None] * len(legs.streams)
+    for dec, g in zip(legs.value_decoders, legs.vgroups):
+        for j, i in enumerate(g):
+            planes[i] = dec.read_planes(j)
+    per_stream = DUMP_BYTES // 4 // len(planes)
+    rng = np.random.default_rng(0)
+    for k, name in enumerate(("y", "cr", "cb")):
+        size = planes[0][k].size
+        pos = np.sort(rng.choice(size, min(size, per_stream * (4 if k == 0 else 1) // 6), replace=False))
+        np.save(os.path.join(directory, f"{prefix}{name}.npy"), np.stack([p[k][pos] for p in planes]).astype(np.float32))
+        np.save(os.path.join(directory, f"{prefix}{name}_positions.npy"), pos.astype(np.float64))
 
 
 def roofline_block(st, peak, peak_src, traffic):
@@ -553,7 +616,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="value leg only (used for the ncu launch list)")
     ap.add_argument("--no-extras", action="store_true", help="skip config_720p / single_stream_1080p")
     ap.add_argument("--no-verify", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write the value leg's decoded pictures (a fixed sample) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = env_int("RANK", 0)
     local_rank = env_int("LOCAL_RANK", 0)
@@ -636,6 +703,8 @@ def main():
             ok = torch.tensor([1.0 if verdict["verified"] and verdict["lane_walk_pictures_equal_pictures"] else 0.0], device="cuda")
             dist.all_reduce(ok, op=dist.ReduceOp.MIN)
             verdict["all_ranks"] = bool(ok.item() > 0.5)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, legs, "" if world == 1 else f"rank{rank}_")
     e_steps = args.steps
     if args.no_e2e:
         e_frames, e_dt, e_st, e_clocks = 0, 1.0, {"h2d_bytes": 0, "d2h_bytes": 0}, None

@@ -8,12 +8,9 @@ for p in (ROOT, os.path.join(ROOT, "tools")):
     if p not in sys.path:
         sys.path.insert(0, p)
 
-REFERENCE = "/root/reference"
-
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box via gpurun)")
-    config.addinivalue_line("markers", "reference: needs the read-only reference tree at /root/reference")
 
 
 def _cuda_problem():
@@ -38,12 +35,8 @@ def _cuda_problem():
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir(REFERENCE)
     gpu_items = [item for item in items if "gpu" in item.keywords]
     problem = _cuda_problem() if gpu_items else None
-    for item in items:
-        if "reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present on this box"))
     for item in gpu_items:
         if problem:  # a plain `pytest tests` on a box without a GPU runs the CPU suite and skips these
             item.add_marker(pytest.mark.skip(reason=f"no usable CUDA device: {problem[:120]}"))

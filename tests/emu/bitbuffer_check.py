@@ -2,16 +2,24 @@
 (through tests/emu/bitbuffer_test.cpp, exact-size malloc) with growing and random writes in both
 modes; every byte the protocol hands out is written, so AddressSanitizer aborts the process on any
 byte the returned pointer does not cover.  Where the REFERENCE's own arithmetic leaves enough room, the
-state (capacity, length, index) must equal that of the compiled reference's bit_buffer_* functions
-(oracle/_ref, src/wasm/buffer.c:48-71, 157-190).  Prints "bitbuffer ok: N writes" on success."""
+state (capacity, length, index, content) must equal that of the reference's bit_buffer_* functions
+(src/wasm/buffer.c:48-71, 157-190).
+
+    bitbuffer_check.py <bitbuffer_test lib> <states.json>             compare with the recorded reference states
+    bitbuffer_check.py <bitbuffer_test lib> <states.json> <ref lib>   run the reference beside it and record them
+
+Prints "bitbuffer ok: N writes" on success."""
 import ctypes
-import os
+import hashlib
+import json
 import sys
 
 import numpy as np
 
 lib = ctypes.CDLL(sys.argv[1])
-ref = ctypes.CDLL(sys.argv[2]) if len(sys.argv) > 2 and os.path.exists(sys.argv[2]) else None
+STATES = sys.argv[2]
+ref = ctypes.CDLL(sys.argv[3]) if len(sys.argv) > 3 else None
+recorded = None if ref is not None else json.load(open(STATES))["trials"]
 lib.bbt_create.restype = ctypes.c_void_p
 lib.bbt_create.argtypes = [ctypes.c_uint, ctypes.c_int]
 lib.bbt_destroy.argtypes = [ctypes.c_void_p]
@@ -48,6 +56,10 @@ def content(t):
     return bytes(lib.bbt_bytes(t)[:length])
 
 
+def trace_digest(states):
+    return hashlib.sha256(repr(states).encode()).hexdigest()[:16]
+
+
 writes = 0
 # the advisor's case: capacity 1000, 900 bytes buffered, then 1500 (the reference sizes the expansion at 2000)
 for mode in (2, 1):
@@ -81,14 +93,16 @@ for mode in (2, 1):
         writes += 1
     lib.bbt_destroy(t)
 
-# random traffic; against the compiled reference wherever the reference itself stays inside its allocation
+# random traffic; against the reference wherever the reference itself stays inside its allocation
 rng = np.random.default_rng(7)
+trials = []
 for trial in range(300):
     mode = int(rng.integers(1, 3))
     cap = int(rng.integers(1, 4000))
     t = lib.bbt_create(cap, mode)
     r = ref.bit_buffer_create(cap, mode) if ref is not None else None
-    in_domain = r is not None
+    in_domain = True
+    states = []  # (capacity, length, index, content digest) after every write inside the reference's domain
     for step in range(int(rng.integers(1, 40))):
         n = int(rng.integers(0, 3000)) if rng.random() < 0.8 else int(rng.integers(0, 40))
         chunk = bytes(rng.integers(0, 256, n, dtype=np.uint8))
@@ -96,7 +110,12 @@ for trial in range(300):
         writes += 1
         cap_t, len_t, idx_t, _ = state(t)
         assert content(t).endswith(chunk) and len_t <= cap_t
-        if in_domain:
+        if in_domain and r is None:
+            if step == recorded[trial]["steps"]:
+                in_domain = False
+            else:
+                states.append((cap_t, len_t, idx_t, hashlib.sha256(content(t)).hexdigest()[:16]))
+        elif in_domain:
             ref.bit_buffer_get_write_ptr(r, n)
             if r.contents.byte_capacity - r.contents.byte_length < n:
                 in_domain = False  # the reference would now write past its allocation: no parity defined from here on
@@ -106,12 +125,21 @@ for trial in range(300):
                 assert (cap_t, len_t, idx_t) == (r.contents.byte_capacity, r.contents.byte_length, r.contents.index), \
                     (trial, step, (cap_t, len_t, idx_t), (r.contents.byte_capacity, r.contents.byte_length, r.contents.index))
                 assert content(t) == bytes(r.contents.bytes[:len_t])
+                states.append((cap_t, len_t, idx_t, hashlib.sha256(content(t)).hexdigest()[:16]))
         # the decoder consumes some of what is buffered
         idx = int(rng.integers(idx_t >> 3, len_t + 1)) << 3
         lib.bbt_set_index(t, idx)
-        if in_domain:
+        if in_domain and r is not None:
             r.contents.index = idx
     lib.bbt_destroy(t)
     if r is not None:
         ref.bit_buffer_destroy(r)
-print("bitbuffer ok:", writes, "writes", "(reference compared)" if ref is not None else "(no reference build)")
+        trials.append({"steps": len(states), "states": trace_digest(states)})
+    else:
+        assert trace_digest(states) == recorded[trial]["states"], \
+            f"trial {trial}: capacity / length / index / content differ from the reference's within its first {len(states)} writes"
+if ref is not None:
+    with open(STATES, "w") as f:
+        json.dump({"trials": trials}, f, indent=0, separators=(",", ":"))
+        f.write("\n")
+print("bitbuffer ok:", writes, "writes", "(reference recorded)" if ref is not None else "(reference compared)")

@@ -1,5 +1,7 @@
 """Shared test helpers: library loading, clip access, oracle record access."""
 import ctypes
+import hashlib
+import json
 import os
 import subprocess
 import sys
@@ -14,6 +16,7 @@ from jsmpeg_b200 import capi, decoder  # noqa: E402
 
 ORACLE_LIB = os.path.join(ROOT, "oracle", "liboracle.so")
 REF_LIB = os.path.join(ROOT, "oracle", "_ref", "libjsmpeg_ref.so")
+REF_GOLDEN = os.path.join(ROOT, "tests", "golden", "reference")
 
 
 class PictureInfo(ctypes.Structure):
@@ -60,9 +63,44 @@ def oracle_lib():
 
 
 def ref_lib():
+    """The compiled reference (oracle/_ref), where tools/make_reference_golden.py records from it; None elsewhere."""
     if not os.path.exists(REF_LIB):
         return None
     return capi.load_library(REF_LIB)
+
+
+def digest(data):
+    """Short content hash (sha256, 64 bits) of bytes or of an array's memory."""
+    if not isinstance(data, (bytes, bytearray)):
+        data = np.ascontiguousarray(data).tobytes()
+    return hashlib.sha256(data).hexdigest()[:16]
+
+
+def record_decode(frames, idx, es=None):
+    """What a reference decode is recorded as in tests/golden/reference/decodes.json."""
+    out = {"index": list(idx), "planes": [[digest(p) for p in f] for f in frames]}
+    if es is not None:
+        out["es"] = digest(es)
+    return out
+
+
+def reference_golden(name):
+    """tests/golden/reference/<name>.json: what the compiled reference computed on the tests' inputs."""
+    with open(os.path.join(REF_GOLDEN, name + ".json")) as f:
+        return json.load(f)
+
+
+def assert_matches_reference(key, frames, idx, es=None, first=0):
+    """frames / bit indices of a decode against the reference's decode of the same stream (decodes.json[key]);
+    idx None: planes only; `first` skips pictures whose planes the C reference leaves uninitialised."""
+    want = reference_golden("decodes")[key]
+    if es is not None:
+        assert digest(es) == want["es"], f"{key}: the input stream is not the one the reference decoded"
+    assert idx is None or list(idx) == want["index"], f"{key}: bit indices differ from the reference"
+    got = [[digest(p) for p in f] for f in frames]
+    assert len(got) == len(want["planes"]), f"{key}: {len(got)} vs {len(want['planes'])} pictures"
+    for k in range(first, len(got)):
+        assert got[k] == want["planes"][k], f"{key}: picture {k} differs from the reference (Y, Cr, Cb digests)"
 
 
 def decode_all(lib, packets, options=None, keep=True, max_frames=None):

@@ -35,29 +35,25 @@ def test_reference_arm_prints_one_contract_line():
 
 
 def test_checker_hash_is_fnv1a64_of_the_planes():
-    """bench.py's `verified` compares hashes made by oracle/ref_bench.c; pin that function to the textbook
-    FNV-1a 64 on a small buffer, and the reference's per-picture hashes to hashes of its own planes."""
-    import ctypes
+    """bench.py's `verified` and the GPU tests compare pictures by FNV-1a 64 of Y | Cr | Cb; pin the function to the
+    textbook FNV-1a 64 on a small buffer, and the hashes of a clip's pictures to the ones the reference's harness
+    (oracle/ref_bench.c: ref_picture_hashes, recorded in tests/golden/reference/picture_hashes.json) gave."""
     import numpy as np
     sys.path.insert(0, helpers.ROOT)
     import bench
-    lib = bench.ref_library()
-    if lib is None:
-        import pytest
-        pytest.skip("oracle/_ref not built")
     data = np.frombuffer(b"jsmpeg_b200 fnv check", dtype=np.uint8).copy()
     h = 1469598103934665603
     for byte in data.tobytes():
         h = ((h ^ byte) * 1099511628211) & 0xFFFFFFFFFFFFFFFF
-    assert lib.ref_hash_bytes(1469598103934665603, data.ctypes.data, data.size) == h
+    assert bench.oracle_library().oracle_hash_bytes(1469598103934665603, data.ctypes.data, data.size) == h
     es = b"".join(p for _, p in helpers.clip_packets(176, 144, 5, seed=3, noise=4))
-    buf = (ctypes.c_uint64 * 8)()
-    n = lib.ref_picture_hashes(es, len(es), buf, 8)
-    assert n == 5
-    frames, _, d = helpers.decode_all(helpers.ref_lib(), [(0, es)])
-    for k, (y, cr, cb) in enumerate(frames):
-        assert bench.fnv1a64_planes(np.ascontiguousarray(y), np.ascontiguousarray(cr), np.ascontiguousarray(cb)) == buf[k]
+    want = helpers.reference_golden("picture_hashes")["176x144x5"]
+    assert helpers.digest(es) == want["es"]
+    frames, _, d = helpers.decode_all(helpers.oracle_lib(), [(0, es)])
+    assert [format(bench.fnv1a64_planes(*f), "016x") for f in frames] == want["fnv1a64"]
     d.destroy()
+    # the last-picture hash bench.py's `verified` computes where the reference build is absent
+    assert bench.oracle_last_hash(bench.oracle_library(), es) == (5, int(want["fnv1a64"][-1], 16))
 
 
 def test_reference_arm_other_ranks_exit_quietly():

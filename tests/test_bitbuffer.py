@@ -1,7 +1,8 @@
 """The host bit buffer's write protocol (jsmpeg_b200/csrc/bitbuffer.h, compiled into the product by
 engine.cu) on the CPU under AddressSanitizer: the returned pointer always covers the requested bytes
 (the reference's own sizing does not: src/wasm/buffer.c:53-57 -- advisor finding of round 1), and the
-state equals the compiled reference's wherever the reference stays inside its allocation."""
+state equals the reference's (recorded in tests/golden/reference/bitbuffer.json) wherever the reference stays inside
+its allocation."""
 import os
 import subprocess
 import sys
@@ -21,5 +22,5 @@ def test_write_protocol_under_asan_and_against_the_reference():
                            "-o", lib, os.path.join(HERE, "emu", "bitbuffer_test.cpp")])
     env = dict(os.environ, LD_PRELOAD=asan, ASAN_OPTIONS="detect_leaks=0")
     r = subprocess.run([sys.executable, os.path.join(HERE, "emu", "bitbuffer_check.py"), lib,
-                        os.path.join(ROOT, "oracle", "_ref", "libjsmpeg_ref.so")], env=env, capture_output=True, text=True, timeout=600)
+                        os.path.join(ROOT, "tests", "golden", "reference", "bitbuffer.json")], env=env, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0 and "bitbuffer ok" in r.stdout, r.stdout[-2000:] + r.stderr[-3000:]

@@ -8,10 +8,9 @@ seeds, 25 pictures each (two GOP boundaries: I pictures at 0, 12, 24), decoded
     pinned host rings,
 
 every checked picture hashed (FNV-1a 64 over Y | Cr | Cb, coded size) against the UNMODIFIED reference C
-(oracle/_ref: src/wasm/mpeg1.c:853-864, 947-995 is the loop it runs) decoding the same stream on the host.
+(src/wasm/mpeg1.c:853-864, 947-995 is the loop it runs) decoding the same stream on the host: its hashes are
+recorded in tests/golden/reference/picture_hashes.json (tools/make_reference_golden.py).
 Round 1 checked five pictures of one 1080p stream; nothing looked at a byte of the benchmarked workload."""
-import ctypes
-import os
 import sys
 import threading
 
@@ -25,36 +24,24 @@ sys.path.insert(0, helpers.ROOT)
 pytestmark = pytest.mark.gpu
 
 STREAMS, PICTURES, W, H = 64, 25, 1920, 1080
+SEEDS = [1234 + i for i in range(STREAMS)]
 
 
 @pytest.fixture(scope="module")
 def workload():
     import bench
-    lib = bench.ref_library()
-    if lib is None:
-        pytest.skip("oracle/_ref/libjsmpeg_ref.so not built")
     old = bench.PICTURES
     bench.PICTURES = PICTURES
     try:
-        seeds = [1234 + i for i in range(STREAMS)]
-        clips = bench.load_streams(seeds, W, H)
+        clips = bench.load_streams(SEEDS, W, H)
     finally:
         bench.PICTURES = old
-    want = np.zeros((STREAMS, PICTURES), dtype=np.uint64)
-    workers = bench.host_cores()["usable"]
-
-    def work(k):
-        for c in range(k, STREAMS, workers):
-            buf = (ctypes.c_uint64 * PICTURES)()
-            n = lib.ref_picture_hashes(clips[c], len(clips[c]), buf, PICTURES)
-            assert n == PICTURES, (c, n)
-            want[c, :] = np.frombuffer(buf, dtype=np.uint64)
-
-    ths = [threading.Thread(target=work, args=(k,)) for k in range(workers)]
-    for t in ths:
-        t.start()
-    for t in ths:
-        t.join()
+    rec = helpers.reference_golden("picture_hashes")[f"{W}x{H}x{PICTURES}"]
+    assert rec["seeds"] == SEEDS
+    bad = [i for i, es in enumerate(clips) if helpers.digest(es) != rec["es"][i]]
+    assert not bad, f"streams {bad[:8]} are not the ones the reference decoded"
+    want = np.array([[int(h, 16) for h in row] for row in rec["fnv1a64"]], dtype=np.uint64)
+    assert want.shape == (STREAMS, PICTURES)
     assert len({int(x) for x in want[:, -1]}) == STREAMS  # 64 distinct clips really are distinct
     return bench, clips, want
 

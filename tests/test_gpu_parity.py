@@ -1,8 +1,8 @@
 """GPU parity: the CUDA path (through the C ABI) against the oracle, bit-exact.
 
 Every test here needs a B200 (``-m gpu``).  The oracle (oracle/liboracle.so, our CPU restatement
-pinned to the reference by tests/test_oracle_vs_reference.py) and, when it was built in the
-build container, the compiled reference itself (oracle/_ref) are the checkers.
+pinned to the reference by tests/test_oracle_vs_reference.py) and the reference's own decodes, recorded in
+tests/golden/reference, are the checkers.
 """
 import ctypes
 
@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 
 import helpers
-from helpers import assert_frames_equal, clip_packets, decode_all, oracle_lib, ref_lib
+from helpers import assert_frames_equal, assert_matches_reference, clip_packets, decode_all, oracle_lib
 from jsmpeg_b200 import capi
 from jsmpeg_b200.batch import OUT_DEVICE, OUT_HOST, BatchDecoder
 
@@ -108,7 +108,7 @@ def test_stage2_reconstruct_matches_oracle_planes(w, h, n):
 @pytest.mark.parametrize("w,h,n", SIZES + [(1920, 1080, 5)])
 def test_reference_abi_whole_clip_bit_exact(w, h, n):
     """write everything, decode() until false: planes and bit indices identical to the oracle
-    (and to the compiled reference when oracle/_ref is present)."""
+    and to the reference (its decode recorded in tests/golden/reference/decodes.json)."""
     packets = clip_packets(w, h, n)
     exp_frames, exp_idx, od = decode_all(oracle_lib(), packets)
     got_frames, got_idx, gd = decode_all(capi.product_library(), packets)
@@ -116,12 +116,7 @@ def test_reference_abi_whole_clip_bit_exact(w, h, n):
     assert_frames_equal(got_frames, exp_frames, "CUDA vs oracle")
     assert (gd.width, gd.height, gd.codedSize, gd.frameRate) == (od.width, od.height, od.codedSize, od.frameRate)
     assert abs(gd.decodedTime - od.decodedTime) < 1e-9
-    ref = ref_lib()
-    if ref is not None:
-        ref_frames, ref_idx, rd = decode_all(ref, packets)
-        assert got_idx == ref_idx
-        assert_frames_equal(got_frames, ref_frames, "CUDA vs compiled reference")
-        rd.destroy()
+    assert_matches_reference(f"ffmpeg/{w}x{h}x{n}", got_frames, got_idx, b"".join(p for _, p in packets))
     od.destroy()
     gd.destroy()
 

@@ -48,8 +48,6 @@ def test_row_sliced_streams_in_one_wave_with_b_pictures():
     through theirs, both beside each other; every picture of every stream against the oracle's hashes."""
     import bench
     from test_b_pictures import FIXTURE_720P
-    if bench.ref_library() is None:
-        pytest.skip("oracle/_ref (the hash helper lives there) not built")
     meta = json.load(open(FIXTURE_720P.replace(".m1v", ".json")))
     es = open(FIXTURE_720P, "rb").read()
     n_streams = 64

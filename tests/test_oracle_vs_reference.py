@@ -1,80 +1,70 @@
-"""Pin the oracle to the reference by RUNNING the reference: oracle/_ref/libjsmpeg_ref.so is the
-unmodified src/wasm/mpeg1.c + buffer.c compiled in place (oracle/Makefile).  Every plane byte of
-every picture and every bit index must agree.  Skipped where the reference build is absent."""
+"""Pin the oracle to the reference: every plane byte of every picture and every bit index must equal what the
+unmodified reference C (src/wasm/mpeg1.c + buffer.c) produced on the same streams.  The reference's results are
+recorded in tests/golden/reference/decodes.json (tools/make_reference_golden.py runs the reference to write it)."""
 import numpy as np
 import pytest
 
 import helpers
 import synth_es
 
-pytestmark = pytest.mark.skipif(helpers.ref_lib() is None, reason="oracle/_ref (compiled reference) not built")
-
 
 @pytest.mark.parametrize("name", sorted(synth_es.CASES))
 def test_synthetic_syntax_corners(name):
     es = synth_es.make_case(name)
-    packets = [(0.0, es)]
-    ref_frames, ref_idx, rd = helpers.decode_all(helpers.ref_lib(), packets)
-    orc_frames, orc_idx, od = helpers.decode_all(helpers.oracle_lib(), packets)
-    assert orc_idx == ref_idx
-    helpers.assert_frames_equal(orc_frames, ref_frames, name)
-    assert len(ref_frames) >= 6
-    rd.destroy()
+    orc_frames, orc_idx, od = helpers.decode_all(helpers.oracle_lib(), [(0.0, es)])
+    helpers.assert_matches_reference(f"synth/{name}", orc_frames, orc_idx, es)
+    assert len(orc_frames) >= 6
     od.destroy()
 
 
-@pytest.mark.parametrize("seed", range(6))
-def test_random_syntax_streams(seed):
-    """Fresh random streams (not the committed ones): all corner knobs on at once."""
+def random_syntax_stream(seed):
     k = synth_es.Knobs(width=int(16 * (2 + seed)), height=int(16 * (1 + seed % 3)) + 2 * seed, pictures=7, gop=3,
                        slices=["one", "rows", "random"][seed % 3], slice_gap_prob=0.2, stuffing_prob=0.2,
                        skip_prob=0.3, f_codes=(1, 2, 3, 4), full_pel_prob=0.3, escape_prob=0.3,
                        custom_matrices=bool(seed & 1), extension_user_data=True, ignored_pictures=bool(seed & 2))
-    es = synth_es.SynthStream(k, 1000 + seed).generate()
-    ref_frames, ref_idx, rd = helpers.decode_all(helpers.ref_lib(), [(0.0, es)])
+    return synth_es.SynthStream(k, 1000 + seed).generate()
+
+
+@pytest.mark.parametrize("seed", range(6))
+def test_random_syntax_streams(seed):
+    """Random streams (not the committed ones): all corner knobs on at once."""
+    es = random_syntax_stream(seed)
     orc_frames, orc_idx, od = helpers.decode_all(helpers.oracle_lib(), [(0.0, es)])
-    assert orc_idx == ref_idx
-    helpers.assert_frames_equal(orc_frames, ref_frames, f"seed {seed}")
-    rd.destroy()
+    helpers.assert_matches_reference(f"random/{seed}", orc_frames, orc_idx, es)
     od.destroy()
 
 
 @pytest.mark.parametrize("w,h,n", [(320, 240, 24), (1280, 720, 6)])
 def test_ffmpeg_clips(w, h, n):
     packets = helpers.clip_packets(w, h, n)
-    ref_frames, ref_idx, rd = helpers.decode_all(helpers.ref_lib(), packets)
     orc_frames, orc_idx, od = helpers.decode_all(helpers.oracle_lib(), packets)
-    assert orc_idx == ref_idx and len(ref_frames) == n
-    helpers.assert_frames_equal(orc_frames, ref_frames, f"{w}x{h}")
-    rd.destroy()
+    assert len(orc_frames) == n
+    helpers.assert_matches_reference(f"ffmpeg/{w}x{h}x{n}", orc_frames, orc_idx, b"".join(p for _, p in packets))
     od.destroy()
 
 
+def decode_streaming(lib, packets):
+    """EVICT mode with a small buffer, write-a-packet / decode-what-is-there, like the reference player's
+    streaming loop (src/player.js:222-229).  Returns (frames, bit index after every decode)."""
+    from jsmpeg_b200 import decoder
+    d = decoder.MPEG1Video({"streaming": True, "videoBufferSize": 64 * 1024, "decodeFirstFrame": False}, lib=lib)
+    rec = decoder.PlaneRecorder()
+    d.connect(rec)
+    trace = []
+    for pts, payload in packets:
+        d.write(pts, [payload])
+        while d.decode():
+            trace.append(d.bufferGetIndex())
+    d.destroy()
+    return rec.frames, trace
+
+
 def test_streaming_evict_mode_matches_reference():
-    """EVICT mode with a small buffer, write-a-packet / decode-what-is-there, like the reference
-    player's streaming loop (src/player.js:222-229): same pictures, same indices."""
+    """EVICT streaming: same pictures, same indices as the reference."""
     packets = helpers.clip_packets(320, 240, 24)
-    opts = {"streaming": True, "videoBufferSize": 64 * 1024, "decodeFirstFrame": False}
-
-    def run(lib):
-        from jsmpeg_b200 import decoder
-        d = decoder.MPEG1Video(opts, lib=lib)
-        rec = decoder.PlaneRecorder()
-        d.connect(rec)
-        trace = []
-        for pts, payload in packets:
-            d.write(pts, [payload])
-            while d.decode():
-                trace.append(d.bufferGetIndex())
-        d.destroy()
-        return rec.frames, trace
-
-    ref_frames, ref_trace = run(helpers.ref_lib())
-    orc_frames, orc_trace = run(helpers.oracle_lib())
-    assert orc_trace == ref_trace
-    # the first picture of each plane set may expose never-written heap bytes in the C reference
-    helpers.assert_frames_equal(orc_frames, ref_frames, "EVICT streaming")
-    assert len(ref_frames) >= 20
+    orc_frames, orc_trace = decode_streaming(helpers.oracle_lib(), packets)
+    helpers.assert_matches_reference("evict/320x240x24", orc_frames, orc_trace, b"".join(p for _, p in packets))
+    assert len(orc_frames) >= 20
 
 
 def test_stats_of_synthetic_cases_cover_the_corners():

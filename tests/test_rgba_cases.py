@@ -123,24 +123,24 @@ def test_hand_computed_colours_follow_from_the_formula():
         assert tuple(int(np.clip(v, 0, 255)) for v in (y + r, y - g, y + b)) == want, (y, cb, cr)
 
 
-def test_flat_picture_decodes_to_the_chosen_samples_in_the_reference():
-    """the construction: the compiled reference decodes the flat picture to exactly the chosen Y / Cb / Cr values"""
-    ref = helpers.ref_lib()
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
-    colours = hand_picture()
-    es = flat_picture_es(46, 30, colours)
-    frames, _, d = helpers.decode_all(ref, [(0, es)])
-    assert len(frames) == 1
-    y, cr, cb = frames[0]
-    Y = y.reshape(32, 48)
+def flat_planes(colours):
+    """The Y / Cr / Cb planes (48x32 coded) that hold exactly the chosen samples of hand_picture()."""
+    Y, Cb, Cr = np.zeros((32, 48), np.uint8), np.zeros((16, 24), np.uint8), np.zeros((16, 24), np.uint8)
     for mb, (y0, y1, y2, y3, vb, vr) in enumerate(colours):
         r0, c0 = (mb // 3) * 16, (mb % 3) * 16
-        assert (Y[r0:r0 + 8, c0:c0 + 8] == y0).all() and (Y[r0:r0 + 8, c0 + 8:c0 + 16] == y1).all()
-        assert (Y[r0 + 8:r0 + 16, c0:c0 + 8] == y2).all() and (Y[r0 + 8:r0 + 16, c0 + 8:c0 + 16] == y3).all()
-        assert (cb.reshape(16, 24)[r0 // 2:r0 // 2 + 8, c0 // 2:c0 // 2 + 8] == vb).all()
-        assert (cr.reshape(16, 24)[r0 // 2:r0 // 2 + 8, c0 // 2:c0 // 2 + 8] == vr).all()
-    d.destroy()
+        Y[r0:r0 + 8, c0:c0 + 8], Y[r0:r0 + 8, c0 + 8:c0 + 16] = y0, y1
+        Y[r0 + 8:r0 + 16, c0:c0 + 8], Y[r0 + 8:r0 + 16, c0 + 8:c0 + 16] = y2, y3
+        Cb[r0 // 2:r0 // 2 + 8, c0 // 2:c0 // 2 + 8] = vb
+        Cr[r0 // 2:r0 // 2 + 8, c0 // 2:c0 // 2 + 8] = vr
+    return Y.ravel(), Cr.ravel(), Cb.ravel()
+
+
+def test_flat_picture_decodes_to_the_chosen_samples_in_the_reference():
+    """the construction: the reference decodes the flat picture to exactly the chosen Y / Cb / Cr values
+    (its decode is recorded in tests/golden/reference/decodes.json)"""
+    colours = hand_picture()
+    es = flat_picture_es(46, 30, colours)
+    helpers.assert_matches_reference("rgba/flat_picture", [flat_planes(colours)], None, es)
 
 
 @pytest.mark.gpu

@@ -1,41 +1,13 @@
 """Pin tools/vlc_tables.py (ISO 11172-2 Annex B form) to the reference's tree tables.
 
-The reference's trees (src/wasm/mpeg1.c:59-680 == src/mpeg1.js:1037-1663) are parsed out of the
-reference source at test time -- nothing is copied into this repo -- and every canonical code is
-walked through them exactly the way read_huffman does (src/wasm/mpeg1.c:1742-1748).
+tools/make_reference_golden.py walks the reference's trees (src/wasm/mpeg1.c:59-680 == src/mpeg1.js:1037-1663) the
+way read_huffman does (src/wasm/mpeg1.c:1742-1748) and records in tests/golden/reference/vlc_trees.json every code
+that reaches a leaf, with the leaf's value, and the reference's constant matrices.
 """
-import os
-import re
-
 import pytest
 
+import helpers
 import vlc_tables as V
-from conftest import REFERENCE
-
-
-def _ref_arrays():
-    src = open(os.path.join(REFERENCE, "src/wasm/mpeg1.c")).read()
-    out = {}
-    for m in re.finditer(r"static const (?:int|uint8_t|float) (\w+)\[\] = \{(.*?)\};", src, re.S):
-        body = re.sub(r"//[^\n]*", "", m.group(2))
-        vals = []
-        for tok in body.replace("\n", " ").split(","):
-            tok = tok.strip()
-            if tok:
-                vals.append(eval(tok))  # tokens are literals like "13*3", "0x0a", "-1"
-        out[m.group(1)] = vals
-    return out
-
-
-def _walk(tree, code):
-    state = 0
-    for i, ch in enumerate(code):
-        state = tree[state + int(ch)]
-        if state < 0:
-            return None, i + 1
-        if tree[state] == 0:
-            return tree[state + 2], i + 1
-    return "incomplete", len(code)
 
 
 @pytest.mark.parametrize("name", sorted(V.ALL_VLC))
@@ -43,23 +15,18 @@ def test_prefix_free(name):
     V.check_prefix_free(V.ALL_VLC[name])
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("name", sorted(V.ALL_VLC))
 def test_codes_match_reference_trees(name):
-    tree = _ref_arrays()[name]
+    tree = helpers.reference_golden("vlc_trees")["trees"][name]
     table = V.ALL_VLC[name]
     for code, value in table.items():
-        got, used = _walk(tree, code)
-        assert used == len(code), (name, code)
-        assert got == value, (name, code, got, value)
+        assert tree["codes"].get(code) == value, (name, code, tree["codes"].get(code), value)
     # same number of leaves => the tables are the same function on all valid codes
-    leaves = sum(1 for i in range(0, len(tree), 3) if tree[i] == 0 and i != 0)
-    assert leaves == len(table), (name, leaves, len(table))
+    assert tree["leaves"] == len(tree["codes"]) == len(table), (name, tree["leaves"], len(table))
 
 
-@pytest.mark.reference
 def test_constant_matrices_match_reference():
-    ref = _ref_arrays()
+    ref = helpers.reference_golden("vlc_trees")["matrices"]
     assert ref["ZIG_ZAG"] == V.ZIG_ZAG
     assert ref["DEFAULT_INTRA_QUANT_MATRIX"] == V.DEFAULT_INTRA_QUANT_MATRIX
     assert ref["DEFAULT_NON_INTRA_QUANT_MATRIX"] == V.DEFAULT_NON_INTRA_QUANT_MATRIX
