@@ -189,6 +189,21 @@ int jsmpeg_b200_debug_parse_picture(const uint8_t *es, uint32_t es_len, uint32_t
 int jsmpeg_b200_debug_reconstruct(int mb_width, int mb_height, const void *hdr, const void *coef,
                                   const uint8_t *fwd_y, const uint8_t *fwd_cr, const uint8_t *fwd_cb,
                                   uint8_t *cur_y, uint8_t *cur_cr, uint8_t *cur_cb);
+/* Stage 2 alone over many pictures of any sizes in ONE launcher call, as the engine makes it (the launcher
+ * splits the tasks into launches of its per-launch maximum).  kind = which kernel: */
+#define JSMPEG_B200_RECON_PLANES 0 /* I/P picture -> planes          */
+#define JSMPEG_B200_RECON_RGBA   1 /* I/P picture -> planes + RGBA   */
+#define JSMPEG_B200_RECON_B      2 /* B picture -> planes            */
+#define JSMPEG_B200_RECON_RGBA_B 3 /* B picture -> planes + RGBA     */
+/* geometry[4 i ..] = mb_width, mb_height, display width, height of task i.  Each task brings host buffers of
+ * the same sizes for all tasks: hdr[i] cap_mb * 16 B, coef[i] cap_mb * 768 B, fwd[i] / bwd[i] / cur[i] plane
+ * sets (Y | Cr | Cb of the task's coded size, contiguous) of cap bytes, at least the plane set + coded width
+ * + 64, and rgba[i] of rgba_cap bytes, at least width * height * 4.  bwd is used by the B kinds, rgba by the
+ * RGBA kinds (either may be NULL otherwise).  Every buffer is copied to the device whole and back whole, so
+ * that whatever a launch wrote anywhere in it comes back.  0 on success, -1 on bad arguments or a CUDA error. */
+int jsmpeg_b200_debug_reconstruct_batch(int kind, int n_tasks, const int32_t *geometry, size_t cap_mb, size_t cap,
+                                        size_t rgba_cap, void *const *hdr, void *const *coef, void *const *fwd,
+                                        void *const *bwd, void *const *cur, void *const *rgba);
 
 /* NULL while the decoder works, else why it is dead (see mpeg1_decoder_create). */
 const char *jsmpeg_b200_decoder_last_error(mpeg1_decoder_t *self);

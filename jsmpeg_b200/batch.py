@@ -55,6 +55,8 @@ _BATCH_ABI = {
     "jsmpeg_b200_debug_parse_picture": (ctypes.c_int, [_VP, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int, ctypes.c_int,
                                                        _VP, _VP, _VP, _VP, _VP]),
     "jsmpeg_b200_debug_reconstruct": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "jsmpeg_b200_debug_reconstruct_batch": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, _VP, ctypes.c_size_t, ctypes.c_size_t,
+                                                           ctypes.c_size_t, _VP, _VP, _VP, _VP, _VP, _VP]),
     "jsmpeg_b200_set_default_device": (None, [ctypes.c_int]),
     "jsmpeg_b200_batch_last_error": (ctypes.c_char_p, [_VP]),
     "jsmpeg_b200_batch_set_option": (ctypes.c_int, [_VP, ctypes.c_char_p, ctypes.c_int]),

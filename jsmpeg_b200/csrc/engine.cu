@@ -1494,4 +1494,70 @@ int jsmpeg_b200_debug_reconstruct(int mb_width, int mb_height, const void *hdr, 
 	}
 }
 
+int jsmpeg_b200_debug_reconstruct_batch(int kind, int n_tasks, const int32_t *geometry, size_t cap_mb, size_t cap,
+                                        size_t rgba_cap, void *const *hdr, void *const *coef, void *const *fwd,
+                                        void *const *bwd, void *const *cur, void *const *rgba) {
+	const bool is_b = kind == JSMPEG_B200_RECON_B || kind == JSMPEG_B200_RECON_RGBA_B;
+	const bool is_rgba = kind == JSMPEG_B200_RECON_RGBA || kind == JSMPEG_B200_RECON_RGBA_B;
+	if (kind < JSMPEG_B200_RECON_PLANES || kind > JSMPEG_B200_RECON_RGBA_B || n_tasks < 1) return -1;
+	for (int i = 0; i < n_tasks; i++) {  // every buffer must hold what the task's own launch may touch
+		const int32_t *g = geometry + 4 * i;
+		const size_t mbw = g[0], mbh = g[1];
+		if (g[0] < 1 || g[1] < 1 || mbw * mbh > cap_mb || mbw * mbh * 384 + mbw * 16 + 64 > cap) return -1;
+		if (is_rgba && (g[2] < 1 || g[3] < 1 || (size_t)g[2] > mbw * 16 || (size_t)g[3] > mbh * 16 ||
+		                (size_t)g[2] * g[3] * 4 > rgba_cap))
+			return -1;
+	}
+	// one allocation per buffer, so that an access past a buffer is an access past an allocation
+	std::vector<void *> allocs;
+	auto alloc_copy = [&](const void *src, size_t bytes) {
+		uint8_t *d = dev_alloc<uint8_t>(bytes);
+		allocs.push_back(d);
+		CUDA_CHECK(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice));
+		return d;
+	};
+	int rc = 0;
+	try {
+		std::vector<ReconTask> tasks(n_tasks);
+		std::vector<uint8_t *> d_bufs;  // per task: hdr, coef, fwd, bwd, cur, rgba (nullptr where unused)
+		for (int i = 0; i < n_tasks; i++) {
+			const int32_t *g = geometry + 4 * i;
+			const size_t ysz = (size_t)g[0] * g[1] * 256, csz = ysz / 4;
+			uint8_t *d_hdr = alloc_copy(hdr[i], cap_mb * sizeof(mb_record_t));
+			uint8_t *d_coef = alloc_copy(coef[i], cap_mb * MB_COEF_INT16 * sizeof(int16_t));
+			uint8_t *d_fwd = alloc_copy(fwd[i], cap);
+			uint8_t *d_bwd = is_b ? alloc_copy(bwd[i], cap) : nullptr;
+			uint8_t *d_cur = alloc_copy(cur[i], cap);
+			uint8_t *d_rgba = is_rgba ? alloc_copy(rgba[i], rgba_cap) : nullptr;
+			d_bufs.insert(d_bufs.end(), {d_hdr, d_coef, d_fwd, d_bwd, d_cur, d_rgba});
+			ReconTask &t = tasks[i];
+			t.hdr = reinterpret_cast<const mb_record_t *>(d_hdr);
+			t.coef = reinterpret_cast<const int16_t *>(d_coef);
+			t.cur = PlaneSet{d_cur, d_cur + ysz, d_cur + ysz + csz};
+			t.fwd = PlaneSet{d_fwd, d_fwd + ysz, d_fwd + ysz + csz};
+			if (is_b) t.bwd = PlaneSet{d_bwd, d_bwd + ysz, d_bwd + ysz + csz};
+			t.mb_width = g[0]; t.mb_size = g[0] * g[1];
+			t.coded_width = g[0] * 16; t.coded_height = g[1] * 16;
+			t.rgba = d_rgba; t.width = g[2]; t.height = g[3];
+		}
+		// one call over all tasks: the launcher splits them into launches and sizes each grid as the engine's calls do
+		if (kind == JSMPEG_B200_RECON_PLANES) launch_reconstruct(tasks.data(), n_tasks, 0);
+		else if (kind == JSMPEG_B200_RECON_RGBA) launch_reconstruct_rgba(tasks.data(), n_tasks, 0);
+		else launch_reconstruct_b(tasks.data(), n_tasks, is_rgba, 0);
+		CUDA_CHECK(cudaGetLastError());
+		CUDA_CHECK(cudaDeviceSynchronize());
+		for (int i = 0; i < n_tasks; i++) {
+			void *const host[6] = {hdr[i], coef[i], fwd[i], is_b ? bwd[i] : nullptr, cur[i], is_rgba ? rgba[i] : nullptr};
+			const size_t bytes[6] = {cap_mb * sizeof(mb_record_t), cap_mb * MB_COEF_INT16 * sizeof(int16_t), cap, cap, cap, rgba_cap};
+			for (int k = 0; k < 6; k++)
+				if (host[k]) CUDA_CHECK(cudaMemcpy(host[k], d_bufs[6 * i + k], bytes[k], cudaMemcpyDeviceToHost));
+		}
+	} catch (const std::exception &e) {
+		fprintf(stderr, "%s\n", e.what());
+		rc = -1;
+	}
+	for (void *p : allocs) cudaFree(p);
+	return rc;
+}
+
 }  // extern "C"

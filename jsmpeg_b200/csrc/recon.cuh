@@ -646,7 +646,8 @@ __device__ __forceinline__ void reconstruct_rgba_block(const PARAMS &params, con
 	if (warp < 2) { b = warp * 2 + (lane & 1); local = lane >> 1; }
 	else { b = 4 + (lane >> 4); local = lane & 15; }
 	const int mb_col = first_mb_col + local;
-	const bool in_picture = mb_col < t.mb_width;
+	// the grid covers the launch's widest and tallest picture: a CTA outside this one's rows or columns only joins the barrier
+	const bool in_picture = mb_col < t.mb_width && mb_row < t.mb_height;
 	uint2 rows[8];
 #pragma unroll
 	for (int r = 0; r < 8; r++) rows[r] = make_uint2(0u, 0u);

@@ -129,6 +129,30 @@ def assert_frames_equal(a, b, what=""):
                                      f"{p[w[:8]]} vs {q[w[:8]]}")
 
 
+def canvas2d_rgba(y, cr, cb, width, height):
+    """numpy restatement of the reference's integer renderer (src/canvas2d.js:53-122); the
+    renderer's `cb` parameter receives the decoder's Cr plane and vice versa (SURVEY Q8)."""
+    cw = ((width + 15) >> 4) << 4
+    Y = y.reshape(-1, cw).astype(np.int32)
+    hw = cw >> 1
+    CR = cr.reshape(-1, hw).astype(np.int32)
+    CB = cb.reshape(-1, hw).astype(np.int32)
+    out = np.full((height, width, 4), 255, np.uint8)
+    cols, rows = width >> 1, height >> 1
+    ccb = CR[:rows, :cols]  # what the renderer calls cb
+    ccr = CB[:rows, :cols]
+    r = (ccb + ((ccb * 103) >> 8)) - 179
+    g = ((ccr * 88) >> 8) - 44 + ((ccb * 183) >> 8) - 91
+    b = (ccr + ((ccr * 198) >> 8)) - 227
+    for dy in range(2):
+        for dx in range(2):
+            yy = Y[dy:rows * 2:2, dx:cols * 2:2]
+            out[dy:rows * 2:2, dx:cols * 2:2, 0] = np.clip(yy + r, 0, 255)
+            out[dy:rows * 2:2, dx:cols * 2:2, 1] = np.clip(yy - g, 0, 255)
+            out[dy:rows * 2:2, dx:cols * 2:2, 2] = np.clip(yy + b, 0, 255)
+    return out
+
+
 def clip_packets(width, height, frames, seed=1234, noise=9):
     import gen_streams
     return gen_streams.make_clip_es(width, height, frames, seed, noise)

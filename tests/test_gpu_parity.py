@@ -241,30 +241,6 @@ def test_partial_picture_then_more_data():
     assert len(exp) == 2 + 3
 
 
-def _canvas2d_rgba(y, cr, cb, width, height):
-    """numpy restatement of the reference's integer renderer (src/canvas2d.js:53-122); the
-    renderer's `cb` parameter receives the decoder's Cr plane and vice versa (SURVEY Q8)."""
-    cw = ((width + 15) >> 4) << 4
-    Y = y.reshape(-1, cw).astype(np.int32)
-    hw = cw >> 1
-    CR = cr.reshape(-1, hw).astype(np.int32)
-    CB = cb.reshape(-1, hw).astype(np.int32)
-    out = np.full((height, width, 4), 255, np.uint8)
-    cols, rows = width >> 1, height >> 1
-    ccb = CR[:rows, :cols]  # what the renderer calls cb
-    ccr = CB[:rows, :cols]
-    r = (ccb + ((ccb * 103) >> 8)) - 179
-    g = ((ccr * 88) >> 8) - 44 + ((ccb * 183) >> 8) - 91
-    b = (ccr + ((ccr * 198) >> 8)) - 227
-    for dy in range(2):
-        for dx in range(2):
-            yy = Y[dy:rows * 2:2, dx:cols * 2:2]
-            out[dy:rows * 2:2, dx:cols * 2:2, 0] = np.clip(yy + r, 0, 255)
-            out[dy:rows * 2:2, dx:cols * 2:2, 1] = np.clip(yy - g, 0, 255)
-            out[dy:rows * 2:2, dx:cols * 2:2, 2] = np.clip(yy + b, 0, 255)
-    return out
-
-
 @pytest.mark.parametrize("name", ["ffmpeg_176x144_ip", "odd_size"])
 def test_rgba_epilogue_matches_canvas2d_formula(name):
     from jsmpeg_b200.batch import OUT_RGBA
@@ -275,7 +251,7 @@ def test_rgba_epilogue_matches_canvas2d_formula(name):
     while bd.decode(1, OUT_RGBA):
         y, cr, cb = bd.read_planes(0)
         got = bd.read_rgba(0)
-        exp = _canvas2d_rgba(y, cr, cb, info["width"], info["height"])
+        exp = helpers.canvas2d_rgba(y, cr, cb, info["width"], info["height"])
         assert np.array_equal(got, exp), f"{name}: RGBA picture {n} differs"
         n += 1
     assert n >= 6

@@ -143,7 +143,6 @@ def test_whole_clip_in_one_call_ends_on_the_right_picture(oracle_b):
 
 
 def test_fused_rgba_epilogue_on_b_pictures(oracle_b):
-    from test_gpu_parity import _canvas2d_rgba
     es = natural_clip()[0]
     exp = decode_all(oracle_b, [(0, es)])[0]
     bd = BatchDecoder(1, decode_b=1)
@@ -152,7 +151,7 @@ def test_fused_rgba_epilogue_on_b_pictures(oracle_b):
     while bd.decode(1, OUT_RGBA):
         y, cr, cb = bd.read_planes(0)
         assert_frames_equal([(y, cr, cb)], [exp[n]], f"picture {n} (RGBA run)")
-        assert np.array_equal(bd.read_rgba(0), _canvas2d_rgba(y, cr, cb, 176, 144)), f"RGBA picture {n} differs"
+        assert np.array_equal(bd.read_rgba(0), helpers.canvas2d_rgba(y, cr, cb, 176, 144)), f"RGBA picture {n} differs"
         n += 1
     assert n == len(exp)
     bd.close()
